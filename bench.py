@@ -3,6 +3,7 @@
 
   python bench.py --gpus N --steps K --warmup W          (N>1: launched under torch.distributed.run)
   python bench.py --impl reference ...                    (the reference algorithm's CPU path: oracle port)
+  python bench.py ... --dump-outputs DIR                  (also write the last timed step's outputs as DIR/<name>.npy)
 
 One JSON line on rank 0.  metric = BASELINE.json's "train-step triplets/sec at 256x832x6lvl": frame
 snippets (target + 4 references) per second through forward + losses + backward + Adam.
@@ -127,6 +128,8 @@ def measure_cfg(cfg, args, dev, rank, local, world, steps, full):
     B = PER_GPU_BATCH
     _say('%s: build trainer (+ parameter broadcast)' % cfg)
     trainer = Trainer(cfg, dev, seed=0)
+    dump = full and bool(args.dump_outputs)
+    init = initial_state(trainer) if dump else None
     hb = host_batches(4, B, seed0=1000 * rank)
     static = [torch.empty_like(t, device=dev) for t in hb[0]]
     for s, h in zip(static, hb[0]):
@@ -145,15 +148,44 @@ def measure_cfg(cfg, args, dev, rank, local, world, steps, full):
     trainer.step(tgt, refs, K, Kinv)
     launches_per_step = _lib.lib().ccb_launch_count() - c0
     use_graph = not args.no_graph
+    graph_aux = {}
     if use_graph:
         _say('%s: capture' % cfg)
-        trainer.capture(tgt, refs, K, Kinv, warmup=1)
+        eager_step = trainer.step
+
+        def step_keeping_aux(*a):
+            # replay() hands back only the loss; the loss terms and network outputs of the step that capture() records
+            # live at fixed addresses that every replay rewrites: keep them for --dump-outputs.  Only the recorded step's,
+            # and detached: a live autograd graph of capture()'s eager warm-up step would keep the parameters' gradient
+            # accumulators bound to the warm-up stream, and the captured backward would then wait on uncaptured work.
+            loss, aux = eager_step(*a)
+            if torch.cuda.is_current_stream_capturing():
+                graph_aux['aux'] = {k: [t.detach() for t in v] if isinstance(v, (list, tuple)) else
+                                    (v.detach() if torch.is_tensor(v) else v) for k, v in aux.items()}
+            return loss, aux
+        trainer.step = step_keeping_aux
+        try:
+            trainer.capture(tgt, refs, K, Kinv, warmup=1)
+        finally:
+            del trainer.step
+        assert 'aux' in graph_aux, 'Trainer.capture() did not record its step through trainer.step: the outputs of the ' \
+                                   'graph are out of reach of --dump-outputs'
 
     def one_step():
         if use_graph:
-            return trainer.replay()
+            return trainer.replay(), graph_aux['aux']
         pyramid.clear()
-        return trainer.step(tgt, refs, K, Kinv)[0]
+        return trainer.step(tgt, refs, K, Kinv)
+
+    def run_steps(n):
+        """n steps between two CUDA events; returns the events and what the last step returned."""
+        a, b, out = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True), (None, None)
+        a.record()
+        for _ in range(n):
+            out = None                                     # the previous step's outputs do not outlive it
+            out = one_step()
+        b.record()
+        return a, b, out
 
     warm = max(args.warmup, 3)
     for _ in range(warm):
@@ -164,14 +196,22 @@ def measure_cfg(cfg, args, dev, rank, local, world, steps, full):
     torch.cuda.synchronize(); cdist.barrier()
     if sampler:
         sampler.start()
-    e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-    e0.record()
-    for _ in range(steps):
-        loss = one_step()
-    e1.record()
+    e0, e1, (loss, aux) = run_steps(steps - 1 if dump else steps)
+    ms_total = 0.0
+    if dump:
+        # The dumped (last) step starts from the seeded initial state, reset outside the timed events: after many steps the
+        # state carries every earlier step's rounding (the warp backward scatters with atomics, deep BatchNorms amplify),
+        # while one step from a fixed state differs between runs or builds only by that step's own rounding.
+        e1.synchronize()
+        ms_total = e0.elapsed_time(e1)
+        reset_state(trainer, init)
+        e0, e1, (loss, aux) = run_steps(1)
     torch.cuda.synchronize(); cdist.barrier()
     clocks = sampler.stop() if sampler else None
-    ms_total = cdist.max_over_ranks(e0.elapsed_time(e1), dev)
+    ms_total = cdist.max_over_ranks(ms_total + e0.elapsed_time(e1), dev)
+    if dump and rank == 0:
+        dump_outputs(args.dump_outputs, trainer, loss, aux)
+    loss = aux = None
     # ---- e2e: host inputs, H2D + D2H inside the timed region ----------------------------------------
     _say('%s: e2e region' % cfg)
     loss_host = torch.empty(1).pin_memory()
@@ -194,7 +234,7 @@ def measure_cfg(cfg, args, dev, rank, local, world, steps, full):
     f0.record()
     for i in range(steps):
         feed(i, i + 1 < steps)                             # prefetch mode: batch i+1 crosses PCIe while step i computes
-        loss = one_step()
+        loss = one_step()[0]
         loss_host.copy_(loss.reshape(1), non_blocking=True)
         torch.cuda.current_stream().synchronize()          # the reference reads loss.item() every step
     f1.record()
@@ -232,7 +272,7 @@ def run_ours(args):
     if world == 1 and not args.no_side_configs:
         for c in ('cfg1', 'cfg2', 'cfg3'):
             if c != args.cfg:
-                side[c] = measure_cfg(c, args, dev, rank, local, world, max(5, min(args.steps, 10)), full=False)
+                side[c] = measure_cfg(c, args, dev, rank, local, world, args.steps, full=False)
     ref_gpu = None
     if world == 1 and not args.no_reference_gpu:
         _say('reference on the GPU')
@@ -274,6 +314,61 @@ def run_ours(args):
         if world == 1 and not args.no_cpu_baseline:
             out['cpu_baseline'] = cpu_baseline(args.cfg, budget_s=25.0)
     return out
+
+
+def _state_tensors(trainer):
+    return [t for net in trainer.nets.values() for t in list(net.parameters()) + list(net.buffers())]
+
+
+def initial_state(trainer):
+    """Copies of the trainer's parameters and buffers as built from the seed, tensor by tensor (the optimiser's flat
+    layout may be re-packed by the first data-parallel step)."""
+    return [t.detach().clone() for t in _state_tensors(trainer)]
+
+
+def reset_state(trainer, init):
+    """Back to initial_state(): parameters and buffers restored, Adam moments and step count zero as after construction."""
+    with torch.no_grad():
+        for t, v in zip(_state_tensors(trainer), init):
+            t.copy_(v)
+        for buf in (trainer.opt.exp_avg, trainer.opt.exp_avg_sq, trainer.opt.state):
+            buf.zero_()
+    trainer.refresh_weights()
+
+
+def dump_outputs(out_dir, trainer, loss, aux, budget=64 * 10 ** 6):
+    """What the last timed step computed, as float32 out_dir/<name>.npy: the loss, the loss terms and network outputs it
+    returns (aux), the parameter gradients of its backward and the BatchNorm statistics it leaves (one flat array per net).
+    The step starts from the seeded initial state (measure_cfg).  At most `budget` bytes in all: every array larger than a
+    common cap keeps a fixed, seeded sample of its flattened elements (the same indices whenever the sizes are the same)."""
+    import numpy as np
+    arrs = {'loss': loss}
+    for k, v in aux.items():
+        if isinstance(v, (list, tuple)):
+            arrs.update({'%s_%d' % (k, i): t for i, t in enumerate(v)})
+        elif torch.is_tensor(v):
+            arrs[k] = v
+    for n, net in trainer.nets.items():
+        arrs['grads_' + n] = torch.cat([(p._ccb_grad if getattr(p, '_ccb_grad', None) is not None else torch.zeros_like(p))
+                                        .reshape(-1) for p in net.parameters()])
+        bufs = [b.reshape(-1) for b in net.buffers() if b.is_floating_point()]
+        if bufs:
+            arrs['buffers_' + n] = torch.cat(bufs)
+    # the largest cap that keeps the total within budget: arrays at or under it are written whole
+    left, cap = (budget - 128 * len(arrs)) // 4, None
+    sizes = sorted(t.numel() for t in arrs.values())
+    for i, n in enumerate(sizes):
+        if n * (len(sizes) - i) > left:
+            cap = left // (len(sizes) - i)
+            break
+        left -= n
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in arrs.items():
+        t = t.detach()
+        if cap is not None and t.numel() > cap:
+            idx = np.sort(np.random.default_rng(0).choice(t.numel(), cap, replace=False))
+            t = t.reshape(-1)[torch.from_numpy(idx).to(t.device)]
+        np.save(os.path.join(out_dir, name + '.npy'), t.float().cpu().numpy())
 
 
 # ---------------------------------------------------------------------------------------------------
@@ -601,7 +696,14 @@ def main():
     ap.add_argument('--no-cpu-baseline', action='store_true')
     ap.add_argument('--no-side-configs', action='store_true', help='skip the cfg1/cfg2 side measurements (N=1)')
     ap.add_argument('--no-reference-gpu', action='store_true', help='skip the reference-PyTorch-on-this-GPU context run (N=1)')
+    ap.add_argument('--dump-outputs', metavar='DIR',
+                    help='write the outputs of the last timed step of --cfg, run from the seeded initial state, as DIR/<name>.npy '
+                         '(rank 0, at most 64 MB)')
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error('--steps must be at least 1')
+    if args.dump_outputs and args.impl != 'ours':
+        ap.error('--dump-outputs writes the outputs of --impl ours')
     # Contract: rank 0 prints ONE JSON line on stdout.  Libraries chat on fd 1 (NCCL prints its version banner there):
     # park the real stdout, point fd 1 at stderr for the duration of the run, write the line to the real one at the end.
     sys.stdout.flush()

@@ -13,6 +13,7 @@ import os
 import sys
 import types
 import warnings
+import zlib
 import numpy as np
 import torch
 
@@ -46,10 +47,39 @@ def npy(t):
     return t.detach().cpu().numpy()
 
 
+PART_BYTES = 900 * 1024      # no fixture file over 1 MB: a larger fixture is stored as name.npz, name.1.npz, ...
+
+
 def save(name, d):
-    path = os.path.join(OUT, name + '.npz')
-    np.savez_compressed(path, **{k: (npy(v) if torch.is_tensor(v) else np.asarray(v)) for k, v in d.items()})
-    print(name, '%.1f KB' % (os.path.getsize(path) / 1024), len(d), 'arrays')
+    arrs = {k: (npy(v) if torch.is_tensor(v) else np.asarray(v)) for k, v in d.items()}
+    write_parts(name, arrs)
+    print(name, len(arrs), 'arrays')
+
+
+def part_path(name, i):
+    return os.path.join(OUT, name + ('.%d' % i if i else '') + '.npz')
+
+
+def write_parts(name, arrs):
+    """Arrays in key order, cut into parts of about PART_BYTES (zlib estimate of the deflated members, which leaves room
+    for the npz headers under 1 MB); tests/util.golden() joins the parts."""
+    parts, size = [{}], 0
+    for k, a in arrs.items():
+        n = len(zlib.compress(a.tobytes()))
+        if n > PART_BYTES:
+            raise ValueError('%s: array %s deflates to %d bytes, more than one part holds; store a strided sample '
+                             '(compact())' % (name, k, n))
+        if parts[-1] and size + n > PART_BYTES:
+            parts.append({})
+            size = 0
+        parts[-1][k] = a
+        size += n
+    for i, p in enumerate(parts):
+        np.savez_compressed(part_path(name, i), **p)
+    i = len(parts)
+    while os.path.exists(part_path(name, i)):          # parts left over from a larger earlier run
+        os.remove(part_path(name, i))
+        i += 1
 
 
 def compact(g, limit=40000, stride=61):

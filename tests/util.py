@@ -8,9 +8,17 @@ _cache = {}
 
 
 def golden(name):
+    """The arrays of one fixture; a fixture over 1 MB is stored in parts name.npz, name.1.npz, ... (make_golden.save)."""
     if name not in _cache:
-        with np.load(os.path.join(GOLDEN, name + '.npz')) as z:
-            _cache[name] = {k: z[k] for k in z.files}
+        d, path, i = {}, os.path.join(GOLDEN, name + '.npz'), 0
+        while True:
+            with np.load(path) as z:
+                d.update({k: z[k] for k in z.files})
+            i += 1
+            path = os.path.join(GOLDEN, '%s.%d.npz' % (name, i))
+            if not os.path.exists(path):
+                break
+        _cache[name] = d
     return _cache[name]
 
 
